@@ -3,6 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload randlanet|pointpillars|kpconv]
     python bench.py --impl reference ...        # the CPU arm (torch port of the reference forward)
+    python bench.py ... --dump-outputs DIR      # also write the outputs of the last timed step as DIR/<name>.npy
 
 Launched by the driver either directly (N = 1) or through torch.distributed.run (one rank
 per GPU, NCCL).  One JSON line on rank 0.  A "step" is one forward pass of the workload's
@@ -132,11 +133,40 @@ def to_dev(x, dev):
     return x
 
 
+DUMP_BYTES = 60 * 10 ** 6      # what --dump-outputs writes in all stays under 64 MB, .npy headers included
+
+
+def take_outputs(names, out):
+    """The step's output tensors as host float32 arrays to be written as <name>.npy.  Larger than DUMP_BYTES together,
+    every output is cut to the same fixed, seeded sample of its flattened elements, and <name>.index.npy (float64)
+    holds the flat indices that were kept."""
+    outs = out if isinstance(out, (tuple, list)) else (out,)
+    assert len(outs) == len(names), (len(outs), names)
+    total = 4 * sum(o.numel() for o in outs)
+    arrays = {}
+    for name, o in zip(names, outs):
+        o = o.detach()
+        if total > DUMP_BYTES:
+            k = o.numel() * DUMP_BYTES // (3 * total)      # 4 bytes of value + 8 of index per kept element
+            idx = np.unique(np.random.default_rng(0).integers(0, o.numel(), k))
+            arrays[name + ".index"] = idx.astype(np.float64)
+            o = o.reshape(-1)[torch.from_numpy(idx).to(o.device)]
+        arrays[name] = o.float().cpu().numpy()
+    return arrays
+
+
+def write_outputs(path, arrays):
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 # ----------------------------------------------------------------------------- workloads
 class RandLAWorkload:
     name = "RandLA-Net forward, SemanticKITTI-shaped batch (clouds of 45 056 pts; total_units below), BASELINE configs[2]"
     short = "randlanet_semantickitti_8x45056"
     manifest = "randlanet_semantickitti.manifest.json"
+    output_names = ("logits",)
 
     default_total = 8
 
@@ -205,6 +235,7 @@ class PointPillarsWorkload:
     name = "PointPillars forward, synthetic KITTI frames (~20 000 pts), BASELINE configs[1]"
     short = "pointpillars_kitti"
     manifest = "pointpillars_kitti.manifest.json"
+    output_names = ("cls", "reg", "dir")
     dense_gflop_per_frame = 68.3   # SECOND + SECONDFPN + head at 496 x 432 (SURVEY.md 8d)
     default_total = 1
 
@@ -272,6 +303,7 @@ class KPConvWorkload:
     name = "KPConv (KPFCNN) forward, S3DIS-shaped clouds (65 536 pts, rooms pre-gridded at 4 cm), BASELINE configs[3]"
     short = "kpconv_s3dis"
     manifest = "kpconv_s3dis.manifest.json"
+    output_names = ("logits",)
     gflop_per_cloud = 90.3   # SURVEY.md 8d (encoder 54.8 + decoder/head 35.5)
     default_total = 4
 
@@ -341,8 +373,10 @@ def run_reference(args, wl):
             wl.cpu_forward(sd, inp)
         t0 = time.perf_counter()
         for _ in range(args.steps):
-            wl.cpu_forward(sd, inp)
+            out = wl.cpu_forward(sd, inp)
         dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        write_outputs(args.dump_outputs, take_outputs(wl.output_names, out))
     v = pts * args.steps / dt / 1e6
     line = dict(metric="M points/s forward", value=round(v, 5), unit="Mpoints/s", n_gpus=args.gpus,
                 steps=args.steps, warmup=args.warmup, ms_per_step=round(1e3 * dt / args.steps, 3),
@@ -460,8 +494,11 @@ def run_b200(args, wl):
     is_rl = hasattr(model, "forward_points")
     graphed = is_rl and hasattr(model, "forward_graphed")
 
+    last_out = [None]
+
     def step_resident():
-        return model.forward_graphed(dev_inp) if graphed else model(dev_inp)
+        last_out[0] = model.forward_graphed(dev_inp) if graphed else model(dev_inp)
+        return last_out[0]
 
     def with_gather(out):
         """Post-batch exchange (object_detection.py:222-233 / SURVEY 8e): all_gather of the per-frame results over NCCL so
@@ -508,6 +545,8 @@ def run_b200(args, wl):
     torch.cuda.cudart().cudaProfilerStop()
     launches = L.lib().o3dml_launch_count() - launches0
     clk = clocks.stop() if rank == 0 else None
+    # copied before any later call can overwrite them (graph replays reuse their output buffers)
+    dumped = take_outputs(wl.output_names, last_out[0]) if args.dump_outputs and rank == 0 else None
     if hasattr(model, "backbone_neck_head"):
         model.backbone_neck_head = orig_bnh      # timers cover the resident region only
     lfa_ms_in_step = None
@@ -716,6 +755,8 @@ def run_b200(args, wl):
                             launch="forward replayed from a CUDA graph" if graphed or dense_timers else "eager launches",
                             numa_node_rank0=numa),
                 clocks=clk, e2e=e2e, gpu_launches=int(launches), roofline=roof, cpu_baseline=cpu, **extra)
+    if dumped is not None:
+        write_outputs(args.dump_outputs, dumped)
     emit(line)
     if dist_on:
         dist.destroy_process_group()
@@ -749,14 +790,18 @@ def main():
                     help="clouds / frames in the whole batch, sharded over the ranks: strong scaling (0 = config default)")
     ap.add_argument("--shape", default="kitti", choices=["kitti", "waymo"], help="pointpillars frame shape")
     ap.add_argument("--no-cpu", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step to DIR/<name>.npy (float32; rank 0's frames; a fixed "
+                         "seeded sample of each output when they exceed 60 MB together, see take_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup < 3 and args.impl == "b200":
         args.warmup = 3
     wl = (RandLAWorkload(args.units or 8) if args.workload == "randlanet" else
           PointPillarsWorkload(args.units or 1, shape=args.shape) if args.workload == "pointpillars" else
           KPConvWorkload(args.units or 4))
     if args.impl == "reference":
-        args.steps = min(args.steps, 50)   # bounded CPU sample: each step is one full-size unit
         run_reference(args, wl)
     else:
         run_b200(args, wl)

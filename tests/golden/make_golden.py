@@ -24,10 +24,26 @@ from oracle import refshim, weights, models_torch as MT, ops as O  # noqa: E402
 from open3d_ml_b200 import synth  # noqa: E402
 
 SEED = 1234
+TAP_CAP = 16 * 1024      # values kept per RandLA-Net tap
 
 
 def sample_idx(n, m, seed):
     return np.sort(np.random.default_rng(seed).choice(n, size=min(m, n), replace=False))
+
+
+def sample_rows(t, cap, seed):
+    """[..., C] -> (indices into its [rows, C] view, those rows): at most `cap` values, so that every fixture file
+    stays under 1 MB."""
+    flat = np.asarray(t).reshape(-1, t.shape[-1])
+    rows = sample_idx(flat.shape[0], max(1, cap // flat.shape[1]), seed)
+    return rows, flat[rows]
+
+
+def sample_flat(t, m, seed):
+    """Any tensor -> (its shape, m indices into the flattened tensor, the values there)."""
+    flat = np.asarray(t).reshape(-1)
+    idx = sample_idx(flat.size, m, seed)
+    return np.array(t.shape), idx, flat[idx]
 
 
 # ------------------------------------------------------------------ RandLA-Net
@@ -71,9 +87,18 @@ def make_randlanet():
     print("randlanet: port vs reference rel err %.3e" % err)
     assert err < 1e-5
     save = dict(logits=out.numpy(), B=B, N=N, seed0=100, weight_seed=SEED)
-    for k, v in taps.items():  # [B,C,N,1] -> [B,N,C]
-        save["tap." + k] = v.squeeze(3).transpose(1, 2).contiguous().numpy()
+    for k, v in taps.items():  # [B,C,N,1] -> [B,N,C], a sample of its B * N rows
+        save["tap." + k + ".rows"], save["tap." + k] = sample_rows(v.squeeze(3).transpose(1, 2).numpy(), TAP_CAP, 4)
     np.savez_compressed(os.path.join(HERE, "randlanet_small.npz"), **save)
+
+    # a second shape and weight seed: one cloud of 1024 points
+    sd = weights.seeded_state_dict(man, 77)
+    net.load_state_dict(sd, strict=True)
+    inp = randla_inputs(1, 1024, 900)
+    with torch.no_grad():
+        out = net(inp)
+    np.savez_compressed(os.path.join(HERE, "randlanet_other_shape.npz"), logits=out.numpy(), B=1, N=1024, seed0=900,
+                        weight_seed=77)
 
 
 def make_randlanet_s3dis():
@@ -186,9 +211,10 @@ def make_pointpillars():
         b.point = f2
         with torch.no_grad():
             o2 = net2(b)
-        np.savez_compressed(os.path.join(HERE, "pointpillars_small.npz"), weight_seed=SEED,
-                            frame_seed=210, frame_size=6000,
-                            cls=o2[0].numpy(), reg=o2[1].numpy(), dir=o2[2].numpy())
+        save = dict(weight_seed=SEED, frame_seed=210, frame_size=6000)
+        for name, o in zip(("cls", "reg", "dir"), o2):    # half of every output
+            save[name + "_shape"], save[name + "_idx"], save[name + "_vals"] = sample_flat(o.numpy(), o.numel() // 2, 5)
+        np.savez_compressed(os.path.join(HERE, "pointpillars_small.npz"), **save)
 
 
 # ------------------------------------------------------------------ KPConv

@@ -16,6 +16,12 @@ def golden(name):
     return np.load(os.path.join(GOLDEN, name), allow_pickle=False)
 
 
+def tap_rows(tap, g, key):
+    """The rows of a [..., C] tap that fixture g keeps for `key` (make_golden.py:sample_rows)."""
+    rows = torch.from_numpy(g["tap.%s.rows" % key]).to(tap.device)
+    return tap.reshape(-1, tap.shape[-1])[rows]
+
+
 def state_dict(manifest_name, seed):
     man, extra = weights.load_manifest(os.path.join(GOLDEN, manifest_name))
     return weights.seeded_state_dict(man, int(seed)), extra

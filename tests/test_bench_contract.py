@@ -6,6 +6,8 @@ import os
 import subprocess
 import sys
 
+import numpy as np
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 KEYS = {"metric", "value", "unit", "n_gpus", "steps", "warmup", "ms_per_step", "higher_is_better", "scaling",
         "vs_baseline", "dtype", "data", "config", "e2e", "cpu_baseline", "impl"}
@@ -32,6 +34,32 @@ def test_reference_arm_prints_one_json_line():
     r = _run([sys.executable, "bench.py", "--impl", "reference", "--steps", "1", "--warmup", "0"])
     assert r.returncode == 0, r.stderr[-2000:]
     _check_line(r.stdout, 1)
+
+
+def test_reference_arm_dumps_the_outputs_of_its_last_step(tmp_path):
+    r = _run([sys.executable, "bench.py", "--impl", "reference", "--steps", "1", "--warmup", "0",
+              "--dump-outputs", str(tmp_path)])
+    assert r.returncode == 0, r.stderr[-2000:]
+    _check_line(r.stdout, 1)
+    assert sorted(os.listdir(tmp_path)) == ["logits.npy"]
+    a = np.load(tmp_path / "logits.npy")
+    assert a.dtype == np.float32 and a.shape == (1, 45056, 19) and np.isfinite(a).all()
+
+
+def test_dumped_outputs_are_a_fixed_sample_under_64_mb():
+    import torch
+    import bench
+    outs = (torch.arange(12_000_000, dtype=torch.float32), torch.arange(6_000_000, dtype=torch.float32).view(1000, 6000))
+    a = bench.take_outputs(("x", "y"), outs)
+    assert sorted(a) == ["x", "x.index", "y", "y.index"]
+    assert sum(v.nbytes for v in a.values()) < 64e6
+    for k in ("x", "y"):
+        assert a[k].dtype == np.float32 and a[k + ".index"].dtype == np.float64
+        assert np.array_equal(a[k], a[k + ".index"])            # arange: every kept value is its own index
+    b = bench.take_outputs(("x", "y"), outs)
+    assert all(np.array_equal(a[k], b[k]) for k in a)
+    small = bench.take_outputs(("z",), torch.ones(3, 4))
+    assert list(small) == ["z"] and small["z"].shape == (3, 4)
 
 
 def test_reference_arm_under_torchrun_rank0_only():
