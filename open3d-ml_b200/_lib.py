@@ -142,9 +142,6 @@ def make_src(data, index=None, index_ld=1, out_rows_per_batch=0, src_rows_per_ba
     return s
 
 
-USE_TC_GEMM = os.environ.get("O3DML_GEMM_TC", "1") != "0"
-
-
 def tf32_round(x):
     """fp32 -> nearest TF32 (10 explicit mantissa bits, ties to even), returned as fp32."""
     u = x.contiguous().view(torch.int32).to(torch.int64) & 0xFFFFFFFF
@@ -233,25 +230,25 @@ def pack_linear(w_kc):
     return PackedWeight(w_kc)
 
 
-TC_MIN_K = int(os.environ.get("O3DML_GEMM_TC_MIN_K", "64"))
+TC_MIN_K = 64
 
 
 def _tc_ok(srcs):
     """Tensor-core kernel only where it pays (K >= TC_MIN_K) and where the operand contract of gemm_tc.cu
     holds: every source 4-channel aligned with 16-byte aligned rows, and every source but the last a
     multiple of 32 channels (a 32-channel k-slice never straddles two sources)."""
-    if not USE_TC_GEMM or sum(s.channels for s in srcs) < TC_MIN_K:
+    if sum(s.channels for s in srcs) < TC_MIN_K:
         return False
     if any(s.channels % 32 for s in srcs[:-1]):
         return False
     return all((s.channels % 4 == 0) and (s.ld % 4 == 0) and (s.data % 16 == 0) for s in srcs)
 
 
-USE_ROW_MLP = os.environ.get("O3DML_ROW_MLP", "1") != "0"
+USE_ROW_MLP = True
 # one-thread-per-row layers need rows >= SMs x 256 x a few to fill the machine: below this the tensor-core kernel
 # (128 rows per CTA, K >= TC_MIN_K) has the shorter critical path (1 cloud per GPU: 11 264 rows = 44 CTAs, 25 us
 # against ~10 us; profiles/r02_launches_randlanet_1cloud.md)
-ROW_MLP_MIN_ROWS = int(os.environ.get("O3DML_ROW_MLP_MIN_ROWS", "40000"))
+ROW_MLP_MIN_ROWS = 40000
 
 
 def _rows_small_ok(srcs, out, ld, co):
@@ -290,6 +287,34 @@ def linear(srcs, weight, out, scale=None, shift=None, residual=None, act=None, s
                                  res_ld, act_code(act), float(slope), ptr(out), ld, co, out_nchw_plane,
                                  stream()))
     return out
+
+
+def graph_replay(cache, key, thunk, device):
+    """Runs thunk() by replaying a CUDA graph captured at the first call with `key`, and returns clones of its
+    outputs (a tensor or a tuple of tensors), since the next replay overwrites the graph's own.  thunk must not
+    synchronise with the host and must reuse its buffers from call to call; key must identify every input address.
+
+    The first call runs thunk() eagerly once: that sizes the cached buffers and makes the one-time
+    cudaFuncSetAttribute calls, neither of which may happen under stream capture.  Then the whole device is
+    synchronised, so that no work of it is in flight while capturing (capturing while the previous batch's all_gather
+    was still running faulted with an illegal address in multi-GPU runs, DESIGN.md section 6), and the capture is
+    thread_local, so that CUDA calls of other threads do not invalidate it.  The cache is emptied when it holds more
+    than 8 graphs."""
+    ent = cache.get(key)
+    if ent is None:
+        thunk()
+        torch.cuda.synchronize(device)
+        graph = torch.cuda.CUDAGraph()
+        n0 = lib().o3dml_launch_count()
+        with torch.cuda.graph(graph, capture_error_mode="thread_local"):
+            out = thunk()
+        if len(cache) > 8:
+            cache.clear()
+        ent = cache[key] = (graph, out, lib().o3dml_launch_count() - n0)
+    graph, out, launches = ent
+    graph.replay()
+    lib().o3dml_launch_count_add(launches)
+    return tuple(o.clone() for o in out) if isinstance(out, tuple) else out.clone()
 
 
 def pack_operand_image_host(w_nk):

@@ -6,7 +6,6 @@ The library has no torch dependency: it is a plain C ABI (include/o3dml_b200.h)
 over CUDA kernels, statically linked against cudart.
 """
 import os
-import shlex
 import subprocess
 import sys
 from concurrent.futures import ThreadPoolExecutor
@@ -21,10 +20,6 @@ DEBUG = (["-DO3DML_DEBUG_NAN"] if os.environ.get("O3DML_DEBUG_NAN") else []) + \
 FLAGS = DEBUG + ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
          "-Xcompiler", "-fPIC,-fvisibility=hidden", "--expt-relaxed-constexpr",
          "-ccbin", "/usr/bin/g++"]
-
-
-# development hook: extra nvcc flags (e.g. -DLTC_EAGER_INDEX) for A/B builds on the GPU box; use with --force
-FLAGS += shlex.split(os.environ.get("O3DML_NVCC_EXTRA", ""))
 
 
 def sources():

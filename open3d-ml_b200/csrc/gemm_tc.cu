@@ -36,7 +36,6 @@
 #include "../../include/o3dml_b200.h"
 #include "common.cuh"
 #include "tc.cuh"
-#include <stdlib.h>
 #include <cuda.h>
 #include <algorithm>
 
@@ -670,16 +669,6 @@ static int gemm_tc_launch_bn(const GemmTcParams& p, unsigned grid_x, cudaStream_
     return O3DML_OK;
 }
 
-// development hook: O3DML_GEMM_LITE = the longest product (in 32-channel k-slices) that runs on the LITE kernels;
-// 0 keeps everything on the one-CTA-per-SM kernels
-static int gt_lite_max_slices() {
-    static const int n = [] {
-        const char* e = getenv("O3DML_GEMM_LITE");
-        return e ? atoi(e) : 16;
-    }();
-    return n;
-}
-
 static int gemm_tc_launch(GemmTcParams& p, const void* wimg, cudaStream_t st) {
     if (p.N <= 0 || p.Cout <= 0) return O3DML_OK;
     O3DML_CHECK(p.Kpad % GT_KS == 0 && p.Kpad >= p.K, "linear_tc: weight image K padding must be a multiple of 32");
@@ -699,7 +688,7 @@ static int gemm_tc_launch(GemmTcParams& p, const void* wimg, cudaStream_t st) {
     // the LITE kernels, two CTAs per SM (GtCfg).  Measured (profiles/r02_gemm_lite.md): threshold 4 / 16 / 64 / none =
     // RandLA-Net 220.0 / 220.4 / 220.3 / 220.3, PointPillars 24.4 / 24.9 / 24.9 / 24.9, KPFCNN 48.8 / 49.1 / 48.6 / 48.1
     // M points/s against 217.1 / 24.0 / 46.5 without; LITE for the convolutions (K = 9 C) loses (PointPillars 24.5).
-    const bool lite = p.mode == 0 && !any_gather && p.Kpad / GT_KS <= gt_lite_max_slices() &&
+    const bool lite = p.mode == 0 && !any_gather && p.Kpad / GT_KS <= 16 &&
                       row_tiles * (p.Npad / (bn == 32 ? 32 : 64)) > gt_num_sms();
     if (lite && bn == 128) bn = 64;
     // a grid that fills less than half of the SMs (PointPillars block 3: 27 x 2 CTAs; one cloud per GPU: 6 - 88)

@@ -15,7 +15,6 @@
 #include "../../include/o3dml_b200.h"
 #include "prims.cuh"
 #include <float.h>
-#include <stdlib.h>
 
 namespace o3dml {
 
@@ -88,7 +87,7 @@ __global__ void grid_bbox_kernel(const float* __restrict__ pts, int64_t n,
 // caller can size the cell arrays without a device->host sync.
 __global__ void grid_setup_kernel(const unsigned* __restrict__ bbox,
                                   const int64_t* __restrict__ splits, int batch, float fixed_cs,
-                                  int k, float knn_cell_scale, GridInfo* __restrict__ info, uint32_t* total_cells) {
+                                  int k, GridInfo* __restrict__ info, uint32_t* total_cells) {
     if (blockIdx.x != 0 || threadIdx.x != 0) return;
     uint32_t base = 0;
     for (int b = 0; b < batch; ++b) {
@@ -111,7 +110,7 @@ __global__ void grid_setup_kernel(const unsigned* __restrict__ bbox,
                 float kk = (float)(k < 4 ? 4 : k);
                 float cs2 = sqrtf(kk * e0 * e1 / (3.14159265f * (float)nb));
                 float cs3 = cbrtf(kk * e0 * e1 * e2 / (4.18879f * (float)nb));
-                cs = fmaxf(knn_cell_scale * fmaxf(cs2, cs3), 1e-6f);
+                cs = fmaxf(fmaxf(cs2, cs3), 1e-6f);
             }
             const double cap = 2.0 * (double)nb + 64.0;
             for (int it = 0; it < 64; ++it) {
@@ -383,13 +382,7 @@ static int grid_build(const float* pts, int64_t np, const int64_t* psplits, cons
     const int T = 256;
     grid_init_kernel<<<ceil_div(batch * 6, T), T, 0, st>>>(g.bbox, batch);
     if (np > 0) grid_bbox_kernel<<<(unsigned)ceil_div<int64_t>(np, T), T, 0, st>>>(pts, np, psplits, batch, g.bbox);
-    // cell edge of the k-NN grid relative to the radius expected to hold k points (O3DML_KNN_CELL_SCALE: tuning hook)
-    static const float cell_scale = [] {
-        const char* e = getenv("O3DML_KNN_CELL_SCALE");
-        const float v = e ? (float)atof(e) : 1.0f;
-        return v > 0.1f && v < 10.f ? v : 1.0f;
-    }();
-    grid_setup_kernel<<<1, 32, 0, st>>>(g.bbox, psplits, batch, fixed_cs, k, cell_scale, g.info, g.total_cells);
+    grid_setup_kernel<<<1, 32, 0, st>>>(g.bbox, psplits, batch, fixed_cs, k, g.info, g.total_cells);
     O3DML_CUDA(cudaMemsetAsync(g.cell_start, 0, (g.max_cells + 1) * 4, st));
     O3DML_CUDA(cudaMemsetAsync(g.cursor, 0, (g.max_cells + 1) * 4, st));
     if (np > 0) grid_count_kernel<<<(unsigned)ceil_div<int64_t>(np, T), T, 0, st>>>(pts, np, psplits, batch, g.info, g.cell_of, g.cell_start);

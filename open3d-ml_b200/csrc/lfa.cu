@@ -22,7 +22,6 @@
 // variant plugs into the same tiles.
 #include "../../include/o3dml_b200.h"
 #include "common.cuh"
-#include <stdlib.h>
 #include <string.h>
 
 namespace o3dml {
@@ -283,186 +282,35 @@ static int lfa_launch(const LfaParams& p, cudaStream_t st) {
 
 
 // ---------------------------------------------------------------------------------------------
-// d_out = 16 (the first, largest level: N points x 16 neighbours, 8 + 8 channels).  The tiled
-// kernel above keeps ~2.2 KB of shared memory per point, i.e. <= 12 warps per SM, and at this
-// width the gathers (not the FMAs) are what has to be hidden.  Here one THREAD owns one
-// neighbour row end to end in registers (encoding -> lse1 [-> lse2] -> 16 scores, weights
-// read as warp-uniform LDS.128), and only the [16 rows x 16 channels] scores / features of a
-// point cross shared memory once, channel-major, for the softmax over the neighbours.
-// 256 threads = 16 points; 35 KB of shared memory and <= 64 registers -> 4 CTAs (32 warps) per SM.
+// d_out = 16 (the first, largest level: N points x 16 neighbours, 8 + 8 channels) in the model.  The tiled
+// kernel above keeps ~2.2 KB of shared memory per point, i.e. <= 12 warps per SM, and at this width the
+// gathers (not the FMAs) are what has to be hidden.  Here one THREAD owns one neighbour row end to end in
+// registers (encoding -> lse1 [-> lse2] -> 16 scores), and only the [16 rows x 16 channels] scores /
+// features of a point cross shared memory once, channel-major, for the softmax over the neighbours.
+// 256 threads = 16 points, 34 KB of shared memory.
+//
+// The layer's weights travel in the KERNEL PARAMETER block (constant bank 0): every FFMA takes its weight as
+// a c[0][imm] operand, so no instruction and no register-file write is spent on loading weights.  (Read from
+// shared memory as warp-uniform LDS.128, they cost 440 cycles of shared-memory return path per warp against
+// 206 issue cycles: such a kernel is bound by the broadcast writes, not by the FMAs.)  The host passes the
+// packed weights from HOST memory.
 constexpr int L16_PTS = 16;                 // points per CTA pass
 constexpr int L16_ROWS = L16_PTS * LFA_K;   // 256 rows = threads
 constexpr int L16_RS = L16_ROWS + 4;        // channel-major row stride (conflict-free LDS.128)
+constexpr int L16C_CTAS = 5;                // resident CTAs per SM the register allocation is held to (42 registers)
 
-template <int STAGE>
-__global__ void __launch_bounds__(L16_ROWS, 4)
-lfa16_kernel(const __grid_constant__ LfaParams p, int64_t num_groups) {
-    constexpr int D = 16, H = 8;
-    __shared__ __align__(16) float W10[12 * H];        // [10][8] + scale + shift
-    __shared__ __align__(16) float Wl2[H * H + 2 * H];  // [8][8] + scale + shift (stage 2)
-    __shared__ __align__(16) float Ws[D * D + D];       // [16][16] + bias
-    __shared__ __align__(16) float St[D * L16_RS];      // scores, channel-major
-    __shared__ __align__(16) float Xs[D * L16_RS];      // X, channel-major
-    const int tid = threadIdx.x;
-    for (int i = tid; i < 10 * H; i += L16_ROWS) W10[i] = p.w10t[i];
-    if (tid < H) {
-        W10[10 * H + tid] = p.s10[tid];
-        W10[11 * H + tid] = p.t10[tid];
-        if (STAGE == 2) {
-            Wl2[H * H + tid] = p.s2[tid];
-            Wl2[H * H + H + tid] = p.t2[tid];
-        }
-    }
-    if (STAGE == 2 && tid < H * H) Wl2[tid] = p.wl2t[tid];
-    Ws[tid] = p.wst[tid];
-    if (tid < D) Ws[D * D + tid] = p.bs[tid];
-    __syncthreads();
-
-    const int pl = tid >> 4, j = tid & 15;
-    for (int64_t grp = blockIdx.x; grp < num_groups; grp += gridDim.x) {
-        const int64_t g = grp * L16_PTS + pl;
-        float x[D];
-#pragma unroll
-        for (int c = 0; c < D; ++c) x[c] = 0.f;
-        float r1[H];
-#pragma unroll
-        for (int o = 0; o < H; ++o) r1[o] = 0.f;
-        if (g < p.total) {
-            const int64_t b = g / p.n_per_batch;
-            const int64_t gn = b * p.n_per_batch + load_index(p.nidx, g * LFA_K + j, p.nidx_is64);
-            const float4 f0 = *reinterpret_cast<const float4*>(p.feat + (size_t)gn * H);
-            const float4 f1 = *reinterpret_cast<const float4*>(p.feat + (size_t)gn * H + 4);
-            const float qx = p.coords[3 * g], qy = p.coords[3 * g + 1], qz = p.coords[3 * g + 2];
-            const float cx = p.coords[3 * gn], cy = p.coords[3 * gn + 1], cz = p.coords[3 * gn + 2];
-            const float dx = qx - cx, dy = qy - cy, dz = qz - cz;
-            float e[10];
-            e[0] = sqrtf(__fadd_rn(__fadd_rn(__fmul_rn(dx, dx), __fmul_rn(dy, dy)), __fmul_rn(dz, dz)));
-            e[1] = dx; e[2] = dy; e[3] = dz;
-            e[4] = qx; e[5] = qy; e[6] = qz;
-            e[7] = cx; e[8] = cy; e[9] = cz;
-            x[0] = f0.x; x[1] = f0.y; x[2] = f0.z; x[3] = f0.w;
-            x[4] = f1.x; x[5] = f1.y; x[6] = f1.z; x[7] = f1.w;
-#pragma unroll
-            for (int q = 0; q < 10; ++q) {
-                const float4 wa = *reinterpret_cast<const float4*>(&W10[q * H]);
-                const float4 wb = *reinterpret_cast<const float4*>(&W10[q * H + 4]);
-                r1[0] = fmaf(e[q], wa.x, r1[0]); r1[1] = fmaf(e[q], wa.y, r1[1]);
-                r1[2] = fmaf(e[q], wa.z, r1[2]); r1[3] = fmaf(e[q], wa.w, r1[3]);
-                r1[4] = fmaf(e[q], wb.x, r1[4]); r1[5] = fmaf(e[q], wb.y, r1[5]);
-                r1[6] = fmaf(e[q], wb.z, r1[6]); r1[7] = fmaf(e[q], wb.w, r1[7]);
-            }
-#pragma unroll
-            for (int o = 0; o < H; ++o) {
-                const float a = fmaf(r1[o], W10[10 * H + o], W10[11 * H + o]);
-                r1[o] = a >= 0.f ? a : 0.2f * a;
-            }
-            if (STAGE == 1) {
-#pragma unroll
-                for (int o = 0; o < H; ++o) x[H + o] = r1[o];
-            } else {
-                float r2[H];
-#pragma unroll
-                for (int o = 0; o < H; ++o) r2[o] = 0.f;
-#pragma unroll
-                for (int k = 0; k < H; ++k) {
-                    const float4 wa = *reinterpret_cast<const float4*>(&Wl2[k * H]);
-                    const float4 wb = *reinterpret_cast<const float4*>(&Wl2[k * H + 4]);
-                    r2[0] = fmaf(r1[k], wa.x, r2[0]); r2[1] = fmaf(r1[k], wa.y, r2[1]);
-                    r2[2] = fmaf(r1[k], wa.z, r2[2]); r2[3] = fmaf(r1[k], wa.w, r2[3]);
-                    r2[4] = fmaf(r1[k], wb.x, r2[4]); r2[5] = fmaf(r1[k], wb.y, r2[5]);
-                    r2[6] = fmaf(r1[k], wb.z, r2[6]); r2[7] = fmaf(r1[k], wb.w, r2[7]);
-                }
-#pragma unroll
-                for (int o = 0; o < H; ++o) {
-                    const float a = fmaf(r2[o], Wl2[H * H + o], Wl2[H * H + H + o]);
-                    x[H + o] = a >= 0.f ? a : 0.2f * a;
-                }
-            }
-        }
-        // scores of this row
-        float sc[D];
-#pragma unroll
-        for (int c = 0; c < D; ++c) sc[c] = Ws[D * D + c];
-#pragma unroll
-        for (int k = 0; k < D; ++k) {
-#pragma unroll
-            for (int c4 = 0; c4 < D; c4 += 4) {
-                const float4 w = *reinterpret_cast<const float4*>(&Ws[k * D + c4]);
-                sc[c4 + 0] = fmaf(x[k], w.x, sc[c4 + 0]);
-                sc[c4 + 1] = fmaf(x[k], w.y, sc[c4 + 1]);
-                sc[c4 + 2] = fmaf(x[k], w.z, sc[c4 + 2]);
-                sc[c4 + 3] = fmaf(x[k], w.w, sc[c4 + 3]);
-            }
-        }
-#pragma unroll
-        for (int c = 0; c < D; ++c) {
-            St[c * L16_RS + tid] = sc[c];
-            Xs[c * L16_RS + tid] = x[c];
-        }
-        __syncthreads();
-        // thread (pl, c = j): softmax over the 16 neighbour rows of channel c
-        {
-            const float* srow = St + j * L16_RS + pl * LFA_K;
-            const float* xrow = Xs + j * L16_RS + pl * LFA_K;
-            float4 s4[4];
-#pragma unroll
-            for (int q = 0; q < 4; ++q) s4[q] = *reinterpret_cast<const float4*>(srow + 4 * q);
-            float m = s4[0].x;
-#pragma unroll
-            for (int q = 0; q < 4; ++q) m = fmaxf(fmaxf(fmaxf(m, s4[q].x), s4[q].y), fmaxf(s4[q].z, s4[q].w));
-            float num = 0.f, den = 0.f;
-#pragma unroll
-            for (int q = 0; q < 4; ++q) {
-                const float4 xv = *reinterpret_cast<const float4*>(xrow + 4 * q);
-                const float e0 = expf(s4[q].x - m), e1 = expf(s4[q].y - m);
-                const float e2 = expf(s4[q].z - m), e3 = expf(s4[q].w - m);
-                den += (e0 + e1) + (e2 + e3);
-                num = fmaf(e0, xv.x, num);
-                num = fmaf(e1, xv.y, num);
-                num = fmaf(e2, xv.z, num);
-                num = fmaf(e3, xv.w, num);
-            }
-            if (g < p.total) p.agg[(size_t)g * D + j] = num / den;
-        }
-        __syncthreads();
-    }
-}
-
-template <int STAGE>
-static int lfa16_launch(const LfaParams& p, cudaStream_t st) {
-    const int64_t groups = ceil_div<int64_t>(p.total, L16_PTS);
-    int dev = 0, sms = 148;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    const int64_t cap = (int64_t)sms * 4;   // resident CTAs; each walks groups with a grid stride
-    const unsigned blocks = (unsigned)(groups < cap ? groups : cap);
-    lfa16_kernel<STAGE><<<blocks, L16_ROWS, 0, st>>>(p, groups);
-    O3DML_LAUNCH_CHECK();
-    o3dml_count_launches(1);
-    return O3DML_OK;
-}
-
-// Same kernel with the layer's weights in the KERNEL PARAMETER block (constant bank 0): every
-// FFMA takes its weight as a c[0][imm] operand, so no instruction and no register-file write
-// is spent on loading weights.  (ncu on lfa16_kernel: 110 warp-uniform LDS.128 per row =
-// 440 cycles of shared-memory return path per warp vs 206 issue cycles -> that kernel is bound
-// by the broadcast writes, not by the FMAs.)  The host passes the packed weights from HOST memory.
 struct alignas(16) Lfa16W {
     float v[O3DML_LFA16_WEIGHT_FLOATS];
 };
 constexpr int W16_W10 = 0, W16_S10 = 80, W16_T10 = 88, W16_WL2 = 96, W16_S2 = 160, W16_T2 = 168,
               W16_WS = 176, W16_BS = 432;
 
-// PF = gather pipelining over the groups a CTA walks (the un-pipelined kernel spent 23 % of its stall samples on the
-// two dependent round trips index -> coordinates / features, profiles/r02_lfa_stalls.md):
-//   0  none            1  the neighbour index of the next group is requested one group ahead (raw word, common.cuh)
-//   2  index two groups ahead, coordinates + feature row of the next group one group ahead (14 more registers:
-//      4 CTAs per SM instead of 5)
-#ifndef L16C_CTAS
-#define L16C_CTAS 5    // resident CTAs per SM the register allocation is held to (42 registers)
-#endif
-template <int STAGE, int PF>
-__global__ void __launch_bounds__(L16_ROWS, PF == 2 ? 4 : L16C_CTAS)
+// Each CTA walks groups of 16 points with a grid stride, and the neighbour index of its next group is
+// requested one group ahead, kept as a raw loaded word until that group comes up (common.cuh): the two
+// dependent round trips index -> coordinates / feature row were 23 % of the stall samples without it
+// (profiles/r02_lfa_stalls.md).
+template <int STAGE>
+__global__ void __launch_bounds__(L16_ROWS, L16C_CTAS)
 lfa16c_kernel(const __grid_constant__ LfaParams p, const __grid_constant__ Lfa16W w, int64_t num_groups) {
     constexpr int D = 16, H = 8;
     __shared__ __align__(16) float St[D * L16_RS];      // scores, channel-major
@@ -476,13 +324,10 @@ lfa16c_kernel(const __grid_constant__ LfaParams p, const __grid_constant__ Lfa16
     const unsigned ngrp = (unsigned)num_groups, gstride = gridDim.x;
     const int* nidx32 = reinterpret_cast<const int*>(p.nidx);
     const int ishift = p.nidx_is64 ? 1 : 0;
-    // pipeline state: (base, raw) of the group whose index is in flight, (gn, data) of the group whose rows are
+    // (base, raw) of the group whose neighbour index is in flight
     int raw_a = 0;
     unsigned base_a = 0;
     bool ok_a = false;
-    int gn_b = -1;
-    float4 fb0 = make_float4(0.f, 0.f, 0.f, 0.f), fb1 = fb0;
-    float qb[6] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
     auto request_index = [&](unsigned grp_) {
         const unsigned g_ = grp_ * L16_PTS + pl;
         ok_a = grp_ < ngrp && g_ < total;
@@ -491,24 +336,7 @@ lfa16c_kernel(const __grid_constant__ LfaParams p, const __grid_constant__ Lfa16
             raw_a = nidx32[((size_t)g_ * LFA_K + j) << ishift];   // stays a raw loaded word until its group comes up
         }
     };
-    auto request_rows = [&](unsigned grp_) {     // consumes the index requested for grp_
-        gn_b = ok_a ? (int)(base_a + (unsigned)raw_a) : -1;
-        if (gn_b >= 0) {
-            const unsigned g_ = grp_ * L16_PTS + pl;
-            const float* fr = p.feat + (size_t)(unsigned)gn_b * H;
-            fb0 = *reinterpret_cast<const float4*>(fr);
-            fb1 = *reinterpret_cast<const float4*>(fr + 4);
-            const float* cq = p.coords + (size_t)g_ * 3;
-            const float* cn = p.coords + (size_t)(unsigned)gn_b * 3;
-            qb[0] = cq[0]; qb[1] = cq[1]; qb[2] = cq[2];
-            qb[3] = cn[0]; qb[4] = cn[1]; qb[5] = cn[2];
-        }
-    };
-    if (PF >= 1) request_index(blockIdx.x);
-    if (PF == 2) {
-        request_rows(blockIdx.x);
-        request_index(blockIdx.x + gstride);
-    }
+    request_index(blockIdx.x);
     for (unsigned grp = blockIdx.x; grp < ngrp; grp += gstride) {
         const unsigned g = grp * L16_PTS + pl;
         float x[D];
@@ -517,18 +345,8 @@ lfa16c_kernel(const __grid_constant__ LfaParams p, const __grid_constant__ Lfa16
         int gn = -1;
         float4 f0 = make_float4(0.f, 0.f, 0.f, 0.f), f1 = f0;
         float qx = 0.f, qy = 0.f, qz = 0.f, cx = 0.f, cy = 0.f, cz = 0.f;
-        if (PF == 2) {
-            gn = gn_b;
-            f0 = fb0; f1 = fb1;
-            qx = qb[0]; qy = qb[1]; qz = qb[2]; cx = qb[3]; cy = qb[4]; cz = qb[5];
-            request_rows(grp + gstride);                 // next group: rows in flight from here
-            request_index(grp + 2 * gstride);            // the one after: index
-        } else if (g < total) {
-            if (PF == 1) {
-                gn = (int)(base_a + (unsigned)raw_a);
-            } else {
-                gn = (int)(g - g % npb) + nidx32[((size_t)g * LFA_K + j) << ishift];
-            }
+        if (g < total) {
+            gn = (int)(base_a + (unsigned)raw_a);
             const float* fr = p.feat + (size_t)(unsigned)gn * H;
             f0 = *reinterpret_cast<const float4*>(fr);
             f1 = *reinterpret_cast<const float4*>(fr + 4);
@@ -537,7 +355,7 @@ lfa16c_kernel(const __grid_constant__ LfaParams p, const __grid_constant__ Lfa16
             qx = cq[0]; qy = cq[1]; qz = cq[2];
             cx = cn[0]; cy = cn[1]; cz = cn[2];
         }
-        if (PF == 1) request_index(grp + gstride);
+        request_index(grp + gstride);
         if (gn >= 0) {
             const float dx = qx - cx, dy = qy - cy, dz = qz - cz;
             float e[10];
@@ -623,34 +441,15 @@ lfa16c_kernel(const __grid_constant__ LfaParams p, const __grid_constant__ Lfa16
     }
 }
 
-template <int STAGE, int PF>
-static int lfa16c_launch_pf(const LfaParams& p, const Lfa16W& w, cudaStream_t st) {
+template <int STAGE>
+static int lfa16c_launch(const LfaParams& p, const Lfa16W& w, cudaStream_t st) {
     const int64_t groups = ceil_div<int64_t>(p.total, L16_PTS);
-    const int64_t cap = (int64_t)device_sm_count() * (PF == 2 ? 4 : L16C_CTAS);
+    const int64_t cap = (int64_t)device_sm_count() * L16C_CTAS;
     const unsigned blocks = (unsigned)(groups < cap ? groups : cap);
-    lfa16c_kernel<STAGE, PF><<<blocks, L16_ROWS, 0, st>>>(p, w, groups);
+    lfa16c_kernel<STAGE><<<blocks, L16_ROWS, 0, st>>>(p, w, groups);
     O3DML_LAUNCH_CHECK();
     o3dml_count_launches(1);
     return O3DML_OK;
-}
-
-// development hook: O3DML_LFA16_PF = 0 | 1 | 2 selects the gather pipelining depth (default below)
-static int lfa16_pf_mode() {
-    static const int mode = [] {
-        const char* e = getenv("O3DML_LFA16_PF");
-        const int m = e ? atoi(e) : 1;
-        return m < 0 ? 0 : m > 2 ? 2 : m;
-    }();
-    return mode;
-}
-
-template <int STAGE>
-static int lfa16c_launch(const LfaParams& p, const Lfa16W& w, cudaStream_t st) {
-    switch (lfa16_pf_mode()) {
-        case 0: return lfa16c_launch_pf<STAGE, 0>(p, w, st);
-        case 2: return lfa16c_launch_pf<STAGE, 2>(p, w, st);
-        default: return lfa16c_launch_pf<STAGE, 1>(p, w, st);
-    }
 }
 
 }  // namespace o3dml
@@ -683,8 +482,8 @@ extern "C" int o3dml_randla_lfa_pool(int stage, int d, const float* coords, cons
 #define LFA_CASE(DD)                                                              \
     case DD:                                                                      \
         return stage == 1 ? lfa_launch<DD, 1>(p, st) : lfa_launch<DD, 2>(p, st);
-    if (d == 16) return stage == 1 ? lfa16_launch<1>(p, st) : lfa16_launch<2>(p, st);
     switch (d) {
+        LFA_CASE(16)
         LFA_CASE(32)
         LFA_CASE(64)
         LFA_CASE(128)

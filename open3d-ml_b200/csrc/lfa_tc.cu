@@ -273,11 +273,7 @@ lfa_pool_tc_kernel(const __grid_constant__ LfaTcParams p) {
     // with two CTAs per SM the wait is where the other CTA gets the issue slots and the shared-memory port.
     constexpr bool PREF = D >= 64;
     constexpr bool LATE = C::STREAM;
-#ifdef LTC_RAW_INDEX_ALL
-    constexpr bool RAW_INDEX = true;
-#else
     constexpr bool RAW_INDEX = C::STREAM;
-#endif
     constexpr int FCH = PREF ? (H / 8) / NPART : 1;      // feature chunks (8 channels) per thread
     int64_t g_nx = p.total, nb_nx = -1, g_n2 = p.total, base_n2 = -1;
     RawIndex raw_n2 = {0, 0};

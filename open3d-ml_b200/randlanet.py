@@ -36,15 +36,13 @@ def _fold_bn(sd, prefix, bias=None, eps=BN_EPS):
 
 
 class RandLANetB200:
-    def __init__(self, state_dict, num_layers=4, num_neighbors=16, device=None, use_tc=None,
-                 sub_sampling_ratio=None, use_graph=None):
+    def __init__(self, state_dict, num_layers=4, num_neighbors=16, device=None, sub_sampling_ratio=None,
+                 use_graph=True):
         L.require_cuda()
-        import os
         self.sub_sampling_ratio = list(sub_sampling_ratio or [4] * num_layers)
-        self.use_graph = (os.environ.get("O3DML_RL_GRAPH", "1") != "0") if use_graph is None else bool(use_graph)
+        self.use_graph = bool(use_graph)
         self._graphs = {}
         self._splits = {}
-        self.use_tc = (os.environ.get("O3DML_LFA_TC", "1") != "0") if use_tc is None else bool(use_tc)
         self.device = torch.device(device or "cuda")
         self.num_layers = num_layers
         self.k = num_neighbors
@@ -124,14 +122,13 @@ class RandLANetB200:
         self.in_channels = sd["fc0.weight"].shape[1]
         self._buf = {}
         # ---- fused tail (rl_tail.cu): last decoder layer + fc1 stack chained through tensor memory
-        self.use_tail = os.environ.get("O3DML_RL_TAIL", "1") != "0"
         self.tail = None
         pl = "decoder.%d" % (num_layers - 1)
         wd = sd[pl + ".conv.weight"][:, :, 0, 0]                          # ConvTranspose2d [in, out]
         w0, w1, w3 = (sd["fc1.%d.conv.weight" % j][:, :, 0, 0].t() for j in (0, 1, 3))
         skip_c = 2 * self.d_out[0]
-        if self.use_tail and L.lib().o3dml_randla_tail_supported(skip_c, wd.shape[0] - skip_c, wd.shape[1], w0.shape[1],
-                                                                 w1.shape[1], self.num_classes):
+        if L.lib().o3dml_randla_tail_supported(skip_c, wd.shape[0] - skip_c, wd.shape[1], w0.shape[1], w1.shape[1],
+                                               self.num_classes):
             img = L.pack_tail_image([wd, w0, w1, w3], [32, 64, 32, 32]).to(dev)
             sc, sh = torch.ones(4, 64), torch.zeros(4, 64)
             for li, name in enumerate((pl, "fc1.0", "fc1.1")):
@@ -141,11 +138,11 @@ class RandLANetB200:
             self.tail = (img, sc.contiguous(), sh.contiguous())
 
     # ------------------------------------------------------------------ buffers
-    def _get(self, name, rows, ch):
-        key = (name, rows, ch)
+    def _get(self, name, shape, dtype=torch.float32):
+        key = (name, tuple(shape), dtype)
         t = self._buf.get(key)
         if t is None:
-            t = torch.empty((rows, ch), dtype=torch.float32, device=self.device)
+            t = torch.empty(shape, dtype=dtype, device=self.device)
             self._buf[key] = t
         return t
 
@@ -156,7 +153,7 @@ class RandLANetB200:
     def _lfa_pool(self, stage, d, coords, nidx, feat, B, N, p, agg):
         w = self.w
         pool = "pool1" if stage == 1 else "pool2"
-        if self.use_tc and d in TC_DIMS:
+        if d in TC_DIMS:
             L.check(L.lib().o3dml_randla_lfa_pool_tc(
                 stage, d, L.ptr(coords), L.ptr(nidx), 1 if nidx.dtype == torch.int64 else 0, self.k,
                 L.ptr(feat), B, N, L.ptr(w[p + ".lse1.mlp.wt"]), L.ptr(w[p + ".lse1.mlp.s"]),
@@ -167,7 +164,7 @@ class RandLANetB200:
                 L.ptr(w[p + ".lse2.mlp.t"]) if stage == 2 else None,
                 L.ptr(w["%s.%s.score.img" % (p, pool)]), L.ptr(agg), L.stream()))
             return
-        if d == 16 and self.use_tc:
+        if d == 16:
             L.check(L.lib().o3dml_randla_lfa16_pool(
                 stage, L.ptr(coords), L.ptr(nidx), 1 if nidx.dtype == torch.int64 else 0, self.k,
                 L.ptr(feat), B, N, w["%s.lfa16.%d" % (p, stage)].data_ptr(), L.ptr(agg), L.stream()))
@@ -199,7 +196,7 @@ class RandLANetB200:
         inp = self.to_device(inputs)
         feats = inp["features"]
         B, N0, cin = feats.shape
-        x = self._get("fc0", B * N0, self.w["fc0.wt"].shape[1])
+        x = self._get("fc0", (B * N0, self.w["fc0.wt"].shape[1]))
         L.linear([L.make_src(feats.view(B * N0, cin))], self.w["fc0.wt"], x, self.w["fc0.s"],
                  self.w["fc0.t"], act="leaky", slope=0.2)
         skips = []
@@ -212,14 +209,14 @@ class RandLANetB200:
             N = coords.shape[1]
             rows = B * N
             cflat = coords.view(rows, 3)
-            f1 = self._mlp(p + ".mlp1", [L.make_src(x)], self._get(p + ".f1", rows, h))
-            agg1 = self._get(p + ".agg1", rows, d)
+            f1 = self._mlp(p + ".mlp1", [L.make_src(x)], self._get(p + ".f1", (rows, h)))
+            agg1 = self._get(p + ".agg1", (rows, d))
             self._lfa_pool(1, d, cflat, nidx, f1, B, N, p, agg1)
-            p1 = self._mlp(p + ".pool1.mlp", [L.make_src(agg1)], self._get(p + ".p1", rows, h))
-            agg2 = self._get(p + ".agg2", rows, d)
+            p1 = self._mlp(p + ".pool1.mlp", [L.make_src(agg1)], self._get(p + ".p1", (rows, h)))
+            agg2 = self._get(p + ".agg2", (rows, d))
             self._lfa_pool(2, d, cflat, nidx, p1, B, N, p, agg2)
-            p2 = self._mlp(p + ".pool2.mlp", [L.make_src(agg2)], self._get(p + ".p2", rows, d))
-            enc = self._get(p + ".enc", rows, 2 * d)
+            p2 = self._mlp(p + ".pool2.mlp", [L.make_src(agg2)], self._get(p + ".p2", (rows, d)))
+            enc = self._get(p + ".enc", (rows, 2 * d))
             L.linear([L.make_src(p2), L.make_src(x)], self.w[p + ".out.wt"], enc, None,
                      self.w[p + ".out.t"], act="leaky", slope=0.01)
             if taps is not None:
@@ -227,7 +224,7 @@ class RandLANetB200:
                 taps[p] = enc.view(B, N, 2 * d)
             sub = inp["sub_idx"][i]
             ns = sub.shape[1]
-            pooled = self._get(p + ".sub", B * ns, 2 * d)
+            pooled = self._get(p + ".sub", (B * ns, 2 * d))
             L.check(L.lib().o3dml_gather_max(L.ptr(enc), rows, 2 * d, 2 * d, L.ptr(sub),
                                              1 if sub.dtype == torch.int64 else 0, B * ns,
                                              sub.shape[2], ns, N, 0, L.ptr(pooled), 2 * d,
@@ -237,7 +234,7 @@ class RandLANetB200:
             skips.append((pooled, ns))
             x = pooled
         nlast = skips[-1][1]
-        x = self._mlp("mlp", [L.make_src(x)], self._get("mlp", x.shape[0], x.shape[1]))
+        x = self._mlp("mlp", [L.make_src(x)], self._get("mlp", x.shape))
         ncoarse = nlast
         use_tail = self.tail is not None and taps is None
         for i in range(self.num_layers):
@@ -254,15 +251,15 @@ class RandLANetB200:
                     0.2, self.num_classes, L.ptr(logits), L.stream()))
                 return logits.view(B, N0, self.num_classes)
             cout = self.w[p + ".wt"].shape[1]
-            out = self._get(p, B * nup, cout)
+            out = self._get(p, (B * nup, cout))
             self._mlp(p, [L.make_src(skip),
                           L.make_src(x, index=interp.view(-1), index_ld=1, out_rows_per_batch=nup,
                                      src_rows_per_batch=ncoarse)], out)
             if taps is not None:
                 taps[p] = out.view(B, nup, cout)
             x, ncoarse = out, nup
-        y = self._mlp("fc1.0", [L.make_src(x)], self._get("fc1.0", x.shape[0], 64))
-        y = self._mlp("fc1.1", [L.make_src(y)], self._get("fc1.1", x.shape[0], 32))
+        y = self._mlp("fc1.0", [L.make_src(x)], self._get("fc1.0", (x.shape[0], 64)))
+        y = self._mlp("fc1.1", [L.make_src(y)], self._get("fc1.1", (x.shape[0], 32)))
         logits = torch.empty((B * N0, self.num_classes), dtype=torch.float32, device=self.device)
         self._mlp("fc1.3", [L.make_src(y)], logits, act=None)
         return logits.view(B, N0, self.num_classes)
@@ -281,27 +278,13 @@ class RandLANetB200:
     def _knn(self, points, queries, k, ps, qs, name):
         """o3dml_knn_search into cached int32 buffers (global row ids), no host synchronisation."""
         nq = queries.shape[0]
-        idx = self._geti(name, nq, k)
+        idx = self._get(name, (nq, k), torch.int32)
         batch = ps.numel() - 1
         wsb = L.lib().o3dml_knn_workspace_bytes(points.shape[0], nq, batch)
-        ws = self._getb(name + ".ws", wsb)
+        ws = self._get(name + ".ws", (wsb,), torch.uint8)
         L.check(L.lib().o3dml_knn_search(L.ptr(points), points.shape[0], L.ptr(ps), L.ptr(queries), nq,
                                          L.ptr(qs), batch, k, L.ptr(idx), 0, None, L.ptr(ws), wsb, L.stream()))
         return idx
-
-    def _geti(self, name, rows, cols):
-        key = (name, rows, cols, "i32")
-        t = self._buf.get(key)
-        if t is None:
-            t = self._buf[key] = torch.empty((rows, cols), dtype=torch.int32, device=self.device)
-        return t
-
-    def _getb(self, name, nbytes):
-        key = (name, nbytes, "u8")
-        t = self._buf.get(key)
-        if t is None:
-            t = self._buf[key] = torch.empty((nbytes,), dtype=torch.uint8, device=self.device)
-        return t
 
     def build_pyramid(self, points):
         """The index pyramid of RandLANet.transform (randlanet.py:218-229: per level k-NN of the cloud in
@@ -319,9 +302,9 @@ class RandLANetB200:
             rs = self._row_splits(B, n)
             nb = self._knn(flat, flat, self.k, rs, rs, "pyr.nb.%d" % i)
             ns = n // self.sub_sampling_ratio[i]
-            sub = self._get("pyr.sub.%d" % i, B * ns, 3).view(B, ns, 3)
+            sub = self._get("pyr.sub.%d" % i, (B * ns, 3)).view(B, ns, 3)
             sub.copy_(pc[:, :ns])
-            pool = self._geti("pyr.pool.%d" % i, B * ns, self.k)
+            pool = self._get("pyr.pool.%d" % i, (B * ns, self.k), torch.int32)
             pool.view(B, ns, self.k).copy_(nb.view(B, n, self.k)[:, :ns])
             up = self._knn(sub.view(B * ns, 3), flat, 1, self._row_splits(B, ns), rs, "pyr.up.%d" % i)
             out["coords"].append(flat.view(1, B * n, 3))
@@ -349,26 +332,7 @@ class RandLANetB200:
         if not self.use_graph:
             return thunk()
         key = (name,) + tuple((t.data_ptr(), tuple(t.shape), t.dtype) for t in tensors)
-        ent = self._graphs.get(key)
-        if ent is None:
-            import os
-            legacy = os.environ.get("O3DML_GRAPH_LEGACY") == "1"      # debugging hook: the round-2 first version
-            thunk()                                        # sizes the cached buffers, sets kernel attributes
-            if legacy:
-                torch.cuda.current_stream().synchronize()
-            else:
-                torch.cuda.synchronize(self.device)        # nothing of this device in flight while capturing
-            graph = torch.cuda.CUDAGraph()
-            n0 = L.lib().o3dml_launch_count()
-            with torch.cuda.graph(graph, capture_error_mode="global" if legacy else "thread_local"):
-                out = thunk()
-            if len(self._graphs) > 8:
-                self._graphs.clear()
-            ent = self._graphs[key] = (graph, out, L.lib().o3dml_launch_count() - n0)
-        graph, out, launches = ent
-        graph.replay()
-        L.lib().o3dml_launch_count_add(launches)
-        return out.clone()
+        return L.graph_replay(self._graphs, key, thunk, self.device)
 
     def forward_graphed(self, inputs):
         """forward() for DEVICE-resident inputs, replayed from a CUDA graph keyed by their addresses."""
